@@ -2,7 +2,7 @@
 """Benchmark of the BCNN VGG-16 448x448 train step (BASELINE.json metric) on N B200s, one process per GPU.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload bcnn_s2|bcnn_s1|cbcnn8192|mpn] [--batch 32]
-                  [--impl native|reference]
+                  [--impl native|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).
   value         device-timed images/s, inputs resident in HBM (CUDA events, max over ranks)
@@ -387,6 +387,37 @@ def eager_gpu_bcnn(stage, B, steps):
                      'batch; informational practical bar, not the reference arm')
 
 
+DUMP_SAMPLE = 1 << 15      # elements kept per tensor above this size: --dump-outputs writes ~28 MB for osmenet, less for the rest
+
+
+def _sample(t, seed):
+    """float32 numpy copy of `t`; above DUMP_SAMPLE elements, its flattened elements at DUMP_SAMPLE positions drawn with
+    `seed`, so that two runs (or two builds) keep the same positions."""
+    t = t.detach()
+    if t.numel() > DUMP_SAMPLE:
+        idx = torch.randint(0, t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(seed))
+        t = t.flatten()[idx.to(t.device)]
+    return t.float().cpu().numpy()
+
+
+def dump_outputs(d, outputs, loss, model):
+    """Writes what the last timed step handed its caller as d/<name>.npy: the model outputs (`outputs.npy`, or
+    `outputs_<i>.npy` for a tuple), `loss.npy`, and the state after the optimizer step: `state.npy` (every floating-point
+    state_dict entry, i.e. updated parameters and running statistics) and `grads.npy` (every parameter gradient), each the
+    concatenation in state_dict / named_parameters order of per-tensor samples (_sample, seeded by position)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    outs = outputs if isinstance(outputs, (tuple, list)) else (outputs,)
+    arrays = {'outputs' if len(outs) == 1 else f'outputs_{i}': _sample(o, i) for i, o in enumerate(outs)}
+    arrays['loss'] = _sample(loss, 0)
+    arrays['state'] = np.concatenate([_sample(v, i).ravel() for i, v in enumerate(model.state_dict().values())
+                                      if v.is_floating_point()])
+    arrays['grads'] = np.concatenate([_sample(p.grad, i).ravel() for i, (_, p) in enumerate(model.named_parameters())
+                                      if p.grad is not None])
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + '.npy'), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -403,7 +434,12 @@ def main():
     ap.add_argument('--graph', default='auto', choices=['auto', '0', '1'],
                     help='replay forward+backward from a CUDA graph (Trainer cuda_graph mode); auto = only for the '
                          'host-launch-bound ResNet-50 workload')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs, loss, updated state and gradients of the last timed step to DIR/<name>.npy '
+                         '(float32; tensors above %d elements sampled at seeded positions)' % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.workload is None:
         args.workload = f'bcnn_s{args.stage}'
     if args.impl == 'reference':
@@ -432,7 +468,7 @@ def main():
 
     def step_resident():
         if tr._graph_wanted():           # eager for three steps, captured on the third, replayed from then on
-            _, loss = tr._graph_step(x_dev, y_dev)
+            out, loss = tr._graph_step(x_dev, y_dev)
         else:
             out = tr.model(x_dev)
             loss = tr.criterion(out, y_dev)
@@ -440,7 +476,7 @@ def main():
             loss.backward()
             tr.allreduce.finish()
         tr.optimizer.step()
-        return loss
+        return out, loss
 
     def barrier():
         if world > 1:
@@ -452,27 +488,29 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            res = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return ms.item()
+        return ms.item(), res
 
     warm = max(args.warmup, 5 if use_graph else 3)
     for _ in range(warm):
-        loss = step_resident()
+        _, loss = step_resident()
     torch.cuda.synchronize()
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     _lib.reset_launch_count()
-    ms = timed(step_resident, args.steps)
+    ms, (last_out, last_loss) = timed(step_resident, args.steps)
     launches = _lib.launch_count()
     if use_graph and getattr(tr, '_graph', None) is not None:       # replayed kernels are not seen by the host-side counter
         launches += args.steps * tr._graph['kernels']
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:     # before the e2e leg below trains further (and overwrites graph outputs)
+        dump_outputs(args.dump_outputs, last_out, last_loss, tr.model)
     value = B * world * args.steps / (ms * 1e-3)
 
     # end to end through the public Trainer API with host inputs
@@ -482,7 +520,7 @@ def main():
     else:
         for _ in range(2):
             tr.batch_training(data)
-        ms_e2e = timed(lambda: tr.batch_training(data), args.steps)
+        ms_e2e, _ = timed(lambda: tr.batch_training(data), args.steps)
     e2e = B * world * args.steps / (ms_e2e * 1e-3)
     final_loss = float(loss.item())
 

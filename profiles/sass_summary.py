@@ -1,6 +1,7 @@
 """Per-kernel counts of the SASS mnemonics that prove a Blackwell-native kernel (B200_PROFILING.md): UTC*MMA = tcgen05.mma,
 LDTM/STTM = tcgen05.ld/st, UTMALDG/UTMASTG = TMA tensor load/store (.MULTICAST = cluster multicast), UTCBAR = tcgen05.commit,
-HMMA would be the legacy mma.sync path.  Written to profiles/sass_opcodes.txt by __graft_entry__.build()."""
+HMMA would be the legacy mma.sync path.  Written to profiles/sass_opcodes.txt when run as a script, and to
+hawkeye_b200/build/sass_opcodes.txt by __graft_entry__.build()."""
 import collections
 import os
 import re

@@ -65,3 +65,21 @@ def state_like(module, seed=7):
         else:
             out[k] = det(v.shape, ks, 0.1)
     return out
+
+
+def image_folder(root):
+    """24 random RGB PNGs of growing size in 4 class folders under ``root`` plus the ``<label> <path>`` list the dataset
+    reads; returns the list's path."""
+    import os
+    from PIL import Image
+    rng = np.random.RandomState(0)
+    lines = []
+    for i in range(24):
+        arr = rng.randint(0, 256, size=(40 + i, 50 + 2 * i, 3), dtype=np.uint8)
+        name = f'c{i % 4}/img_{i}.png'
+        os.makedirs(os.path.join(root, f'c{i % 4}'), exist_ok=True)
+        Image.fromarray(arr).save(os.path.join(root, name))
+        lines.append(f'{i % 4} {name}')
+    meta = os.path.join(root, 'train.txt')
+    open(meta, 'w').write('\n'.join(lines) + '\n')
+    return meta

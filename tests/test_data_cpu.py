@@ -1,31 +1,20 @@
 """hawkeye_b200.data — the mirror of the reference's dataset package (dataset/dataset.py, transforms.py:14-73, sampler.py) — on a
-generated image folder: item format, the deterministic eval preset, class-balanced batches; and, when the reference tree is
-importable (here: /root/reference), item-for-item / batch-for-batch equality with the reference's own classes."""
+generated image folder: item format, the deterministic eval preset, class-balanced batches; and item-for-item / batch-for-batch
+equality with what the reference's own classes produced on the same folder (tests/golden/make_golden_compat.py)."""
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
+import detgen
 from hawkeye_b200 import data as D
 
 
 @pytest.fixture(scope='module')
 def folder(tmp_path_factory):
-    from PIL import Image
-    root = tmp_path_factory.mktemp('imgs')
-    rng = np.random.RandomState(0)
-    lines = []
-    for i in range(24):
-        arr = rng.randint(0, 256, size=(40 + i, 50 + 2 * i, 3), dtype=np.uint8)
-        name = f'c{i % 4}/img_{i}.png'
-        os.makedirs(os.path.join(root, f'c{i % 4}'), exist_ok=True)
-        Image.fromarray(arr).save(os.path.join(root, name))
-        lines.append(f'{i % 4} {name}')
-    meta = os.path.join(root, 'train.txt')
-    open(meta, 'w').write('\n'.join(lines) + '\n')
-    return str(root), meta
+    root = str(tmp_path_factory.mktemp('imgs'))
+    return root, detgen.image_folder(root)
 
 
 def test_dataset_items_and_eval_preset(folder):
@@ -55,40 +44,23 @@ def test_balanced_batches(folder):
         assert len(cls) == 2 and (cnt == 3).all()                               # what MAMCLoss needs
 
 
-def _reference_dataset_modules():
-    from oracle import ref_harness as rh
-    if not rh.available():
-        pytest.skip('reference tree not importable')
-    root = rh.find_reference_root()
-    if root not in sys.path:
-        sys.path.insert(0, root)
-    import importlib
-    return (importlib.import_module('dataset.dataset'), importlib.import_module('dataset.transforms'),
-            importlib.import_module('dataset.sampler'))
-
-
 def test_matches_reference_classes(folder):
-    rd, rt, rs = _reference_dataset_modules()
+    G = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_compat.npz'))
     root, meta = folder
     ours = D.FGDataset(root, meta, transform=D.ClassificationPresetEval(crop_size=32, resize_size=36))
-    ref = rd.FGDataset(root, meta, transform=rt.ClassificationPresetEval(crop_size=32, resize_size=36))
-    assert len(ours) == len(ref)
-    for i in (0, 7, 23):
-        a, b = ours[i], ref[i]
-        assert int(a['label']) == int(b['label']) and torch.equal(a['img'], b['img'])
+    assert len(ours) == int(G['data_len'])
+    for j, i in enumerate((0, 7, 23)):
+        a = ours[i]
+        assert int(a['label']) == int(G['data_eval_labels'][j])
+        assert torch.equal(a['img'], torch.from_numpy(G['data_eval_imgs'][j]))
     # train preset: same transform pipeline => same draws from the same torch / python RNG state
     import random
-    to, tr = D.ClassificationPresetTrain(32, auto_augment_policy='ta_wide', random_erase_prob=0.1), \
-        rt.ClassificationPresetTrain(32, auto_augment_policy='ta_wide', random_erase_prob=0.1)
+    to = D.ClassificationPresetTrain(32, auto_augment_policy='ta_wide', random_erase_prob=0.1)
     img = D.default_loader(os.path.join(root, 'c1/img_5.png'))
     torch.manual_seed(11); random.seed(11)
     x = to(img)
-    torch.manual_seed(11); random.seed(11)
-    y = tr(img)
-    assert torch.equal(x, y)
+    assert torch.equal(x, torch.from_numpy(G['data_train_img']))
     # sampler: same numpy call order => same batches
     np.random.seed(5)
     b1 = [list(map(int, b)) for b in D.BalancedBatchSampler(ours, 2, 3)]
-    np.random.seed(5)
-    b2 = [list(map(int, b)) for b in rs.BalancedBatchSampler(ref, 2, 3)]
-    assert b1 == b2 and len(b1) > 0
+    assert b1 == G['data_sampler_batches'].tolist() and len(b1) > 0
